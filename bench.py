@@ -1,6 +1,12 @@
 """bench.py -- headline benchmark of the general_cf training hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload simgcl-amazon]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload simgcl-amazon] [--dump-outputs DIR]
+
+The GPU arm times each training-step loop over K steps after W warm-up steps; the value is the median of five such passes
+of the resident-batch loop.  ``--dump-outputs DIR`` writes what the last step of the last of those passes returned (see
+``outputs_of_step``) once the timed steps are done.  The same arguments give the same graph, weights and batches; the
+backward adds with floating-point atomics, so two runs agree to rounding (amplified in the parameters by Adam's division),
+not bit for bit.
 
 One "step" = one iteration of trainer/trainer.py:63-68 (zero_grad, cal_loss, backward, Adam step) at
 B = 4096 on BASELINE.json configs[1]: SimGCL, d = 64, L = 3, tau = 0.2, on a synthetic graph with the
@@ -79,6 +85,43 @@ def make_batches(rows, cols, n_item, count, seed=2023):
         pick = rs.randint(0, len(rows), size=BATCH)
         out.append(np.stack([rows[pick], cols[pick], rs.randint(0, n_item, size=BATCH)]).astype(np.int64))
     return out
+
+
+DUMP_LIMIT = 64 * 10 ** 6      # bytes of --dump-outputs in all
+DUMP_GRAD_ROWS = 4096          # gradient rows sampled per parameter
+
+
+def outputs_of_step(model, loss, parts):
+    """Host copies of what one training step hands its caller: the loss, every loss term, the parameters after the optimizer
+    step (in full while they fit 3/4 of DUMP_LIMIT, else a seeded sample of rows) and a seeded sample of DUMP_GRAD_ROWS rows of
+    each gradient.  The row samples depend only on the parameter shapes, so two runs with the same arguments pick the same rows."""
+    out = {'loss': loss.detach().float().cpu().numpy()}
+    for k, v in parts.items():
+        out['part_' + k] = torch.as_tensor(v).detach().float().cpu().numpy()
+    named = [(n, p) for n, p in model.named_parameters()]
+    full = sum(p.numel() for _, p in named) * 4 <= DUMP_LIMIT * 3 // 4
+    for i, (n, p) in enumerate(named):
+        x = p.detach().float()
+        if not full and x.dim() > 0 and x.shape[0] > 1:
+            rows = max(1, x.shape[0] * (DUMP_LIMIT * 3 // 4) // (4 * sum(q.numel() for _, q in named)))
+            x = x[torch.from_numpy(np.sort(np.random.RandomState(i).choice(x.shape[0], min(rows, x.shape[0]), replace=False))).to(x.device)]
+        out['param_' + n] = x.cpu().numpy()
+        if p.grad is not None:
+            g = p.grad.detach().float()
+            if g.dim() > 0 and g.shape[0] > DUMP_GRAD_ROWS:
+                g = g[torch.from_numpy(np.sort(np.random.RandomState(1000 + i).choice(g.shape[0], DUMP_GRAD_ROWS, replace=False))).to(g.device)]
+            out['grad_' + n] = g.cpu().numpy()
+    return out
+
+
+def write_outputs(path, arrays):
+    """``path/<name>.npy`` for every array (float32; at most DUMP_LIMIT bytes in all)."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f'--dump-outputs: {total} bytes exceed the {DUMP_LIMIT} byte limit')
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k.replace('/', '_') + '.npy'), np.ascontiguousarray(a, dtype=np.float32))
 
 
 class ClockSampler:
@@ -378,6 +421,8 @@ def run_ours(args):
         model.kmeans.iters = 20                      # the clustering runs once, before the timed region (ncl.py:73-74)
         model._cluster()
 
+    last = {}
+
     def step_resident(i):
         opt.zero_grad()
         b = dev_batches[i % len(dev_batches)]
@@ -386,6 +431,7 @@ def run_ours(args):
         if sync is not None:
             sync.average_gradients(params)
         opt.step()
+        last['loss'], last['parts'] = loss, parts
         return loss
 
     e2e_sampler = [None]
@@ -473,7 +519,8 @@ def run_ours(args):
     passes = sorted((timed(step_resident, no_sampling=True) for _ in range(5)), key=lambda p: p[0])
     ms_res, launches, _ = passes[2]                      # the MEDIAN pass is the value; all five are in timing_log
     ms_res_best = passes[0][0]
-    ms_res_sampled, _, clocks = timed(step_resident, steps=max(K, 60))      # long enough for several NVML samples
+    dump = outputs_of_step(model, last['loss'], last['parts']) if (args.dump_outputs and rank == 0) else None
+    ms_res_sampled, _, clocks = timed(step_resident)
     if clocks is not None:
         clocks['sampled_replay_ms_per_step'] = ms_res_sampled
     # e2e is timed WITHOUT clock sampling (one NVML sample costs ~14 ms of host time, which the per-step
@@ -484,7 +531,7 @@ def run_ours(args):
         ms, _, _ = timed(step_e2e_async, no_sampling=True, tail=lambda: seen.__setitem__(0, seen[0] + len(reader.flush())))
         return ms
     ms_e2e = float(np.median([timed_async() for _ in range(5)]))
-    _, _, clocks_e2e = timed(step_e2e, inline_sampling=True, steps=min(K, 6))
+    _, _, clocks_e2e = timed(step_e2e, inline_sampling=True)
 
     # ---- live kernel timings (CUDA events on the launching stream) over K more steps ----
     engine.TIMER = engine.KernelTimer()
@@ -709,6 +756,9 @@ def run_ours(args):
 
     out = assemble() if rank == 0 else None
     torch.cuda.synchronize()
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
+        del dump
 
     # ---- north_star's partition next to the data-parallel headline: the row-sharded LightGCN step on the config-4 graph
     # family scaled to N/8 (bench_rowshard.py), on every --gpus N line of the default workload ----
@@ -727,7 +777,7 @@ def run_ours(args):
         dog = Watchdog(args.row_shard_deadline, fallback)
         try:
             import bench_rowshard
-            row_shard = bench_rowshard.leg(dist, rank, world, dev, steps=5, warmup=2,
+            row_shard = bench_rowshard.leg(dist, rank, world, dev, steps=K, warmup=W,
                                            log=(lambda m: print('[row_shard] ' + m, file=sys.stderr, flush=True)) if rank == 0 else (lambda m: None))
         except Exception as e:      # noqa: BLE001 -- the leg is an extra record; it must never cost the bench line
             row_shard = {'error': repr(e)[:500]}
@@ -890,7 +940,12 @@ def main():
     ap.add_argument('--row-shard-deadline', type=float, default=420.0, help='seconds after which a wedged row-shard leg is abandoned')
     ap.add_argument('--parallel', default='auto', choices=['auto', 'dp', 'shard'],
                     help='N > 1: dp = one batch per GPU + gradient all-reduce (weak scaling); shard = one batch, table rows sharded')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last timed training step returned (loss, loss terms, updated parameters, a '
+                         'seeded row sample of the gradients) as DIR/<name>.npy, float32, at most 64 MB; same arguments, same inputs')
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != 'ours' or args.workload == 'lightgcn-xl'):
+        raise SystemExit('bench.py: --dump-outputs covers the training step of --impl ours (every workload but lightgcn-xl)')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
     if args.impl == 'reference':
         run_reference(args)

@@ -387,100 +387,47 @@ def test_lean_evaluation_batches_equal_the_dataloader_batches():
     assert isinstance(first, list) and len(first) == 2 and first[1].shape == (64, I)          # the reference's [users, mask] batches untouched
 
 
-def test_vectorised_metrics_match_the_reference_metric_class(tmp_path):
-    """trainer.batch_metric_rows against the reference's own ``Metric.eval_batch`` (trainer/metrics.py:11-80, imported unmodified from oracle/_ref in a
-    subprocess: its config module parses sys.argv at import) on random top-k lists and ground truths, all four metrics."""
-    import json
-    import subprocess
-    import sys
-    ref = os.path.join(ROOT, 'oracle', '_ref')
-    if not os.path.isdir(os.path.join(ref, 'trainer')):
-        import pytest
-        pytest.skip('oracle/_ref not vendored (python oracle/vendor_ref.py in the build container)')
-    body = r'''
-import json, os, sys
-import numpy as np, torch
-ref, root = sys.argv[1], sys.argv[2]
-os.chdir(ref)
-sys.path.insert(0, ref); sys.path.insert(1, root)
-sys.argv = ['main.py', '--model', 'lightgcn', '--device', 'cpu']
-from config.configurator import configs
-configs['test']['metrics'] = ['recall', 'ndcg', 'precision', 'mrr']
-configs['test']['k'] = [5, 20, 40]
-from trainer.metrics import Metric
-rs = np.random.RandomState(5)
-n, n_item, kmax = 300, 500, 40
-top = np.stack([rs.permutation(n_item)[:kmax] for _ in range(n)])
-truths = [rs.choice(n_item, size=rs.randint(1, 50), replace=False).tolist() for _ in range(n)]
-for u in range(n):
-    for _ in range(rs.randint(0, 5)):
-        top[u, rs.randint(0, kmax)] = truths[u][rs.randint(len(truths[u]))]
-want = Metric().eval_batch((torch.from_numpy(top), truths), configs['test']['k'])
-from sslrec_b200.trainer import batch_metric_rows, truth_csr
-import types
-ptr, flat = truth_csr(types.SimpleNamespace(user_pos_lists=truths))
-got = batch_metric_rows(top, np.arange(n), ptr, flat, configs['test']['k'], configs['test']['metrics'])
-print('JSON ' + json.dumps({m: [[float(x) for x in want[m]], [float(x) for x in got[m].sum(0)]] for m in want}))
-'''
-    script = tmp_path / 'ref_metric.py'
-    script.write_text(body)
-    r = subprocess.run([sys.executable, str(script), ref, ROOT], capture_output=True, text=True, timeout=300, cwd=str(tmp_path))
-    lines = [ln for ln in r.stdout.splitlines() if ln.startswith('JSON ')]
-    assert r.returncode == 0 and lines, r.stdout[-1000:] + r.stderr[-2000:]
-    res = json.loads(lines[-1][5:])
-    assert set(res) == {'recall', 'ndcg', 'precision', 'mrr'}
-    for m, (want, got) in res.items():
-        assert np.allclose(want, got, rtol=1e-12, atol=1e-12), (m, want, got)
+def test_vectorised_metrics_match_the_reference_metric_class():
+    """trainer.batch_metric_rows against the reference's own ``Metric.eval_batch`` (trainer/metrics.py:11-80) on random top-k lists and ground
+    truths, all four metrics.  The inputs and the reference's per-k sums are stored in tests/golden/ref_metric_eval_batch.npz
+    (oracle/gen_host_golden.py)."""
+    from sslrec_b200.trainer import batch_metric_rows, truth_csr
+    z = np.load(os.path.join(ROOT, 'tests', 'golden', 'ref_metric_eval_batch.npz'))
+    top, tp, tf = z['top'].astype(np.int64), z['truth_ptr'], z['truth_flat']
+    truths = [tf[tp[u]:tp[u + 1]].tolist() for u in range(top.shape[0])]
+    ks, metrics = [int(k) for k in z['ks']], [str(m) for m in z['metrics']]
+    assert set(metrics) == {'recall', 'ndcg', 'precision', 'mrr'}
+    ptr, flat = truth_csr(types.SimpleNamespace(user_pos_lists=truths))
+    got = batch_metric_rows(top, np.arange(top.shape[0]), ptr, flat, ks, metrics)
+    for m in metrics:
+        want = z['want_' + m]
+        assert np.allclose(want, got[m].sum(0), rtol=1e-12, atol=1e-12), (m, want, got[m].sum(0))
         assert want[-1] > 0
 
 
-def test_host_data_path_reproduces_the_reference_batches_draw_for_draw(tmp_path):
+def test_host_data_path_reproduces_the_reference_batches_draw_for_draw():
     """The reference's own training data path (data_utils/datasets_general_cf.py:6-26 ``PairwiseTrnData`` with its per-pair rejection loop, served by
-    ``DataLoader(trn_data, batch_size, shuffle=True)``, data_handler_general_cf.py:95; imported unmodified from oracle/_ref) against this repository's
-    default host path (vectorised ``sample_negs`` + ``HostBatchLoader``) under the same numpy / torch seeds: identical (user, positive, negative)
-    batches over two epochs -- a graph dense enough that a third of the first draws are rejected."""
-    import json
-    import subprocess
-    import sys
-    ref = os.path.join(ROOT, 'oracle', '_ref')
-    if not os.path.isdir(os.path.join(ref, 'data_utils')):
-        import pytest
-        pytest.skip('oracle/_ref not vendored (python oracle/vendor_ref.py in the build container)')
-    body = r'''
-import json, os, sys
-import numpy as np, scipy.sparse as sp, torch
-import torch.utils.data as tdata
-ref, root = sys.argv[1], sys.argv[2]
-os.chdir(ref)
-sys.path.insert(0, ref); sys.path.insert(1, root)
-sys.argv = ['main.py', '--model', 'lightgcn', '--device', 'cpu']
-from config.configurator import configs
-rs = np.random.RandomState(0)
-U, I = 90, 30
-key = np.unique(rs.randint(0, U, 1500).astype(np.int64) * I + rs.randint(0, I, 1500))
-m = sp.coo_matrix((np.ones(len(key)), (key // I, key % I)), shape=(U, I))
-configs['data']['user_num'], configs['data']['item_num'] = U, I
-from data_utils.datasets_general_cf import PairwiseTrnData as RefData
-from sslrec_b200.data_handler import HostBatchLoader, PairwiseTrnData
-def epochs(ds, loader):
-    np.random.seed(11); torch.manual_seed(12)
-    out = []
-    for _ in range(2):
+    ``DataLoader(trn_data, batch_size, shuffle=True)``, data_handler_general_cf.py:95) against this repository's default host path (vectorised
+    ``sample_negs`` + ``HostBatchLoader``) under the same numpy / torch seeds: identical (user, positive, negative) batches over two epochs and the
+    same generator states afterwards -- a graph dense enough that a third of the first draws are rejected.  The reference's batches and states are
+    stored in tests/golden/ref_pairwise_batches.npz (oracle/gen_host_golden.py)."""
+    from sslrec_b200.data_handler import HostBatchLoader, PairwiseTrnData
+    z = np.load(os.path.join(ROOT, 'tests', 'golden', 'ref_pairwise_batches.npz'))
+    rs = np.random.RandomState(0)
+    U, I = 90, 30
+    key = np.unique(rs.randint(0, U, 1500).astype(np.int64) * I + rs.randint(0, I, 1500))
+    assert int(z['n_user']) == U and int(z['n_item']) == I and np.array_equal(key, z['key'])       # the graph the reference was given
+    m = sp.coo_matrix((np.ones(len(key)), (key // I, key % I)), shape=(U, I))
+    ds = PairwiseTrnData(m)
+    loader = HostBatchLoader(ds, int(z['batch_size']))
+    np.random.seed(11)
+    torch.manual_seed(12)
+    for epoch in range(2):
         ds.sample_negs()
-        out.append([[t.long().tolist() for t in b] for b in loader])
-    return out, np.random.get_state()[1][:8].tolist(), torch.get_rng_state()[:16].tolist()
-a = RefData(m)
-ea = epochs(a, tdata.DataLoader(a, batch_size=128, shuffle=True, num_workers=0))
-b = PairwiseTrnData(m)
-eb = epochs(b, HostBatchLoader(b, 128))
-print('JSON ' + json.dumps({'same_batches': ea[0] == eb[0], 'same_numpy_state': ea[1] == eb[1], 'same_torch_state': ea[2] == eb[2],
-                            'batches': len(ea[0][0]), 'pairs': len(key), 'density': len(key) / (U * I)}))
-'''
-    script = tmp_path / 'ref_data.py'
-    script.write_text(body)
-    r = subprocess.run([sys.executable, str(script), ref, ROOT], capture_output=True, text=True, timeout=600, cwd=str(tmp_path))
-    lines = [ln for ln in r.stdout.splitlines() if ln.startswith('JSON ')]
-    assert r.returncode == 0 and lines, r.stdout[-1000:] + r.stderr[-2000:]
-    res = json.loads(lines[-1][5:])
-    assert res['same_batches'] and res['same_numpy_state'] and res['same_torch_state'], res
-    assert res['batches'] >= 5 and res['density'] > 0.3
+        batches = [[t.long().numpy() for t in b] for b in loader]
+        assert np.array_equal([len(b[0]) for b in batches], z[f'epoch{epoch}_batch_len']), epoch
+        triples = np.stack([np.concatenate([b[i] for b in batches]) for i in range(3)])
+        assert np.array_equal(triples, z[f'epoch{epoch}_triples']), epoch
+    assert np.array_equal(np.random.get_state()[1][:8], z['numpy_state_head'])
+    assert np.array_equal(torch.get_rng_state()[:16].numpy(), z['torch_state_head'])
+    assert len(z['epoch0_batch_len']) >= 5 and len(key) / (U * I) > 0.3
