@@ -122,7 +122,8 @@ SSL_API int ssl_plan_stats(const ssl_plan *plan, int64_t out[4]);
  * edge_mode[v]: 0 keep all; 1 counter-based RNG: keep iff U(seed[v], edge_stream_id, row, col) >= 1-keep
  *               (floor(U + keep), aug_utils.py:28); 2 injected: edge_mask[v][p] != 0, p = CSR
  *               position (rev[p] when transpose).  edge_scale[v] multiplies kept values
- *               (1, or 1/keep for EdgeDrop(resize_val=True), hccf.py:33).
+ *               (1, or 1/keep for EdgeDrop(resize_val=True), hccf.py:33) of a view with edge_mode 1 or 2; a view with
+ *               edge_mode 0 propagates the stored values unscaled.
  * noise_mode[v]: 0 none; 1 RNG uniform(seed[v], noise_stream_id, row, elem);
  *               2 injected: noise_u[v] is a [n_cols, dim] U[0,1) tensor (global row).
  * ------------------------------------------------------------------------------------------ */
@@ -204,13 +205,19 @@ SSL_API int ssl_bpr_bwd(const float *users, int64_t u_stride, const float *items
  *   output (alpha), writes row-major out [n, dim], the K-major tile copy out_t
  *   [ceil(n/64), dim, 64] the streaming side of ssl_softmax_gemm reads (may be NULL),
  *   rinv [n] (the 1/norm used, needed by the backward), and optionally the tf32 split
- *   out_hi = tf32(out), out_lo = out - out_hi, row-major [n, dim] each, plus their transposes
+ *   out_hi = tf32_rna(out), out_lo = tf32_rna(out - out_hi) (cvt.rna: round to nearest, ties away from zero; the 13 low
+ *   mantissa bits of both parts are zero), row-major [n, dim] each, plus their transposes
  *   out_thi / out_tlo [dim, t_pitch] (t_pitch >= ceil64(n), multiple of 4) that
  *   ssl_softmax_gemm_tf32x3 reads through TMA.
  * ssl_softmax_gemm    for every row r of R [n_r, dim] over the rows c of C (row-major C
  *   [n_c, dim] and its K-major tile copy C_t):   e = exp2(R_r . C_c - offset) * colscale[c]
  *   rowsum_part[s, r] = sum_c e   (optional)     o_part[s, r, :] = sum_c e * C_c
- *   for the s-th of n_split contiguous chunks of C.  One launch does the forward of a term
+ *   for the s-th of n_split contiguous chunks of C: chunk s is the 64-row tiles [t0, t1) with t0 = n_ct*s/n_split,
+ *   t1 = n_ct*(s+1)/n_split, n_ct = ceil(n_c/64) (1 <= n_split <= n_ct).  C and C_t are read in whole 64-row tiles: the
+ *   caller supplies ceil64(n_c) rows of C and ceil(n_c/64) tiles of C_t [ceil(n_c/64), dim, 64] (the layout
+ *   ssl_rows_normalize writes), and their padding rows must be finite -- they enter the products and are masked
+ *   afterwards (ssl_rows_normalize writes them as zeros).  R, C, C_t 16-byte aligned; colscale is read for c < n_c
+ *   only.  One launch does the forward of a term
  *   (R = scaled anchors, C = normalised table: log-sum-exp and the softmax-weighted table
  *   average that is the anchor gradient) and, with the roles swapped, its backward
  *   (R = table tile, C = anchors, colscale = g/rowsum: the dense table gradient).

@@ -272,8 +272,6 @@ def _reference_chains_full_predict(case, layer_num, n_users_scored):
     return s
 
 
-@pytest.mark.xfail(strict=False, reason='test.exact_order is an opt-in evaluation mode added after the last GPU run of round 2 (no GPU budget left): '
-                                        'verified by executing its kernel source on the host; this is its first execution on a GPU')
 def test_exact_order_full_predict_reproduces_the_reference_cpu_scores_bit_for_bit():
     from sslrec_b200.config import configs
     g = replay.load_golden('lightgcn', 'small')
